@@ -6,12 +6,19 @@
     python bench.py --mode mpjpe --embed 64 --joints 18 --batch 262144 --scaling strong --gpus N      # configs[2]
     python bench.py --mode train --batch 128 --gpus 8                    # configs[4]: data-parallel training step
     python bench.py --impl reference ...                                 # the reference's own CPU implementation
+    python bench.py ... --dump-outputs DIR                               # also write the last timed step's results
 
 A "step" is one pass of the path over one batch of synthetic sequences.  --mode forward: CISTGCN.forward;
 --mode mpjpe: forward + losses.mpjpe (fused per-frame sums; with N > 1 the 208-byte sums are all-reduced over NCCL
 inside the timed region and both the `[]` and `(0, 2)` reductions are derived).  N > 1: launched by torchrun, one rank
 per GPU.  --scaling weak: every rank owns --batch sequences; strong: --batch is the GLOBAL batch, sharded by rank.
 No collective is on the forward's data path.  Prints ONE JSON line.
+
+--dump-outputs DIR writes what the last timed step returned, as DIR/<name>.npy (float32 / float64), so that two builds
+can be compared output for output: inputs and weights are seeded, so the same arguments give the same inputs.
+forward: pred.npy, the predictions of DUMP_ROWS sequences (a fixed, seeded sample of the batch; all of it when smaller);
+mpjpe: mpjpe_all.npy and mpjpe_per_frame.npy; train: frame_sums.npy and parameters.npy (the flat parameter vector after
+the step).  With N > 1, rank 0 writes its own results.
 """
 import argparse
 import ctypes
@@ -32,6 +39,8 @@ FP32_FMA_PEAK_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12      # CUDA-core FP32 FMA 
 FLOPS_PER_SEQ = {(22, 8): 37.06e6, (22, 16): 40.45e6, (22, 32): 52.22e6, (22, 64): 95.68e6,
                  (18, 8): 29.59e6, (18, 16): 32.32e6, (18, 32): 41.87e6, (18, 64): 77.26e6}
 FPN_FLOPS_PER_SEQ = {22: 29.5e6, 18: 29.5e6 * 18 / 22}
+DUMP_ROWS = 4096            # --dump-outputs: sequences of pred kept (4096 x 25 x 22 x 3 fp32 = 27 MB)
+DUMP_MAX_BYTES = 64 << 20
 
 
 def metric_name(V, mode):
@@ -93,6 +102,32 @@ def fpn_tc_issued_flops_per_seq():
     27 taps + 3 compress slices (2 k-steps) per layer."""
     ksteps_tiles = 2 * ((27 * 1 + 3 * 2) + 3 * (27 * 2 + 3 * 2))
     return ksteps_tiles * 2.0 * 128 * (96 + 32) * 16
+
+
+def _host(t):
+    """t on the host as a float32 / float64 numpy array."""
+    import torch
+    t = t.detach().cpu()
+    return (t if t.dtype == torch.float64 else t.float()).numpy()
+
+
+def _row_sample(t):
+    """A fixed, seeded sample of DUMP_ROWS rows of t (sorted indices), or t itself when it has no more rows."""
+    import torch
+    if t.shape[0] <= DUMP_ROWS:
+        return t
+    idx = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    return t[idx.to(t.device)]
+
+
+def write_dump(d, arrays):
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed {DUMP_MAX_BYTES}")
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -351,6 +386,10 @@ def run_native(args, rank, world, local_rank):
         barrier()
         ms_local = sum(e0.elapsed_time(e1) for e0, e1 in evs)
     ms = max_over_ranks(ms_local)
+    dump = None
+    if args.dump_outputs and rank == 0:                 # before the end-to-end arm runs more steps
+        dump = {"pred": _host(_row_sample(out))} if mode == "forward" else \
+               {"mpjpe_all": _host(out[0]), "mpjpe_per_frame": _host(out[1])}
     NK = _cabi.PROFILE_KINDS
     kms = (ctypes.c_double * NK)()
     kln = (ctypes.c_int64 * NK)()
@@ -523,6 +562,8 @@ def run_native(args, rank, world, local_rank):
         line["result"] = result_note
     if world == 1:
         line["cpu_baseline"] = cpu_baseline(E, V, mode, args.cpu_budget)
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
     sys.stdout.flush()
     os.dup2(saved_stdout, 1)
     print(json.dumps(line), flush=True)
@@ -587,6 +628,9 @@ def run_train(args, rank, world, local_rank):
     barrier()
     ms = max_over_ranks(sum(e0.elapsed_time(e1) for e0, e1 in evs))
     ar_ms = max_over_ranks(sum(a0.elapsed_time(a1) for a0, a1 in ar)) if world > 1 else 0.0
+    dump = None
+    if args.dump_outputs and rank == 0:                 # before the end-to-end arm runs more steps
+        dump = {"frame_sums": _host(sums), "parameters": _host(tr.flat.flat)}
     launches = tr.graph.launches + 1 + (1 if world > 1 else 0)
     clocks = sampler.stop() if rank == 0 else None
     value = world * B * args.steps / (ms / 1e3)
@@ -637,6 +681,8 @@ def run_train(args, rank, world, local_rank):
     }
     if world == 1:
         line["cpu_baseline"] = cpu_baseline(E, V, "train", args.cpu_budget, batch=B)
+    if dump is not None:
+        write_dump(args.dump_outputs, dump)
     sys.stdout.flush()
     os.dup2(saved_stdout, 1)
     print(json.dumps(line), flush=True)
@@ -658,7 +704,10 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="train mode: launch every layer kernel from the host instead of "
                     "replaying the captured CUDA graph of forward + loss + backward")
     ap.add_argument("--cpu-budget", type=float, default=12.0, help="seconds of CPU baseline timing (N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the native path's results; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,4 +1,4 @@
-"""Helpers to read tests/golden/*.npz (written by tests/golden/make_golden.py)."""
+"""Helpers to read tests/golden/*.npz and their taps in tests/golden/taps/ (written by tests/golden/make_golden.py)."""
 import glob
 import os
 
@@ -19,7 +19,8 @@ def load(name):
     E, V, tin, tout, itp = (int(v) for v in d["meta"])
     cfg = O.OracleConfig(input_n=tin, output_n=tout, joints=V, input_gcn=[E] * 4)
     sd = {k[3:]: torch.from_numpy(d[k]) for k in d.files if k.startswith("sd/")}
-    taps = {k[4:]: torch.from_numpy(d[k]) for k in d.files if k.startswith("tap/")}
+    t = np.load(os.path.join(GOLDEN_DIR, "taps", name + ".npz"))
+    taps = {k: torch.from_numpy(t[k]) for k in t.files}
     g = {k: torch.from_numpy(d[k]) for k in ("x", "target", "pred", "mpjpe_all", "mpjpe_frames", "mpjpe_none")}
     g.update(cfg=cfg, sd=sd, taps=taps, interpretable=bool(itp), embed=E)
     return g
@@ -29,3 +30,4 @@ def tol(ref: torch.Tensor, base: float = 1e-4) -> float:
     """fp32 parity bound (SURVEY.md 8c / BASELINE.md section 4): 1e-4 absolute on unit-scale
     outputs, scaled by max(1, |ref|_inf / 4) when the reference output itself is large."""
     return base * max(1.0, float(ref.abs().max()) / 4.0)
+

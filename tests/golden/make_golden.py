@@ -3,8 +3,9 @@
     python tests/golden/make_golden.py
 
 Each file holds: the full reference state_dict ("sd/<key>"), the input x, a target, the
-reference prediction, reference-side taps (Adj / w1 / w2 / ContextLayer attributes read off the
-live module exactly as environment/test.py:146-157 does) and losses.mpjpe values.
+reference prediction and losses.mpjpe values; taps/<name>.npz next to it holds the reference-side
+taps (Adj / w1 / w2 / ContextLayer attributes read off the live module exactly as
+environment/test.py:146-157 does).  Two files keep each one under 1 MB.
 The GPU box has no /root/reference, so these vectors are what pins the oracle there.
 """
 import os
@@ -46,21 +47,24 @@ def main():
                "meta": np.array([E, V, cfg.input_n, cfg.output_n, int(itp)], dtype=np.int64),
                "mpjpe_all": mp(pred, tgt).numpy(), "mpjpe_frames": mp(pred, tgt, reduce_axis=(0, 2)).numpy(),
                "mpjpe_none": mp(pred, tgt, reduce_axis=None).numpy()}
+        taps = {}
         blocks = [(f"st_gcnns.{i}", m) for i, m in enumerate(ref.st_gcnns)] + \
                  [(f"st_gcnns_o.{i}", m) for i, m in enumerate(ref.st_gcnns_o)]
         for p, m in blocks:
-            out[f"tap/{p}.w1"] = m.w1.detach().numpy()
-            out[f"tap/{p}.w2"] = m.w2.detach().numpy()
+            taps[f"{p}.w1"] = m.w1.detach().numpy()
+            taps[f"{p}.w2"] = m.w2.detach().numpy()
             if itp:
-                out[f"tap/{p}.dsgn.Adj"] = m.dsgn.Adj.detach().numpy()
-                out[f"tap/{p}.tsgn.Adj"] = m.tsgn.Adj.detach().numpy()
+                taps[f"{p}.dsgn.Adj"] = m.dsgn.Adj.detach().numpy()
+                taps[f"{p}.tsgn.Adj"] = m.tsgn.Adj.detach().numpy()
         cl = ref.context_layer
         for a in ("joints", "displacements", "seq_joints_n", "seq_joints_dims"):
-            out[f"tap/context_layer.{a}"] = getattr(cl, a).detach().numpy()
+            taps[f"context_layer.{a}"] = getattr(cl, a).detach().numpy()
         for k, v in sd.items():
             out["sd/" + k] = v.numpy()
         path = os.path.join(HERE, name + ".npz")
         np.savez_compressed(path, **out)
+        os.makedirs(os.path.join(HERE, "taps"), exist_ok=True)
+        np.savez_compressed(os.path.join(HERE, "taps", name + ".npz"), **taps)
         print(name, "|pred|max", float(pred.abs().max()), os.path.getsize(path) // 1024, "KiB")
 
 

@@ -2,14 +2,15 @@
 train-mode forward (batch-statistics BatchNorm, running-stat updates), losses.mpjpe with reduce_axis=[], backward
 (every parameter's gradient), Adam; and the eval-mode input gradient.
 
-CPU: the kernels run on the SIMT emulator (tests/emu) and are compared with the UNMODIFIED reference module run by
-PyTorch (needs /root/reference or the vendored oracle/_ref).  GPU (-m gpu): the same comparison through the nvcc-built
+The reference side is _models.OracleModule: the reference model restated by oracle/cistgcn_oracle.py under PyTorch's
+autograd and torch.optim.Adam.  The oracle is pinned to the reference module's outputs in eval mode (tests/golden); in
+train mode it uses torch's batch-statistics BatchNorm (F.batch_norm, training=True), the function nn.BatchNorm calls.
+CPU: the kernels run on the SIMT emulator (tests/emu).  GPU (-m gpu): the same comparison through the nvcc-built
 library on larger shapes."""
 import pytest
 import torch
 
 import _models as M
-import _reference as R
 from cistgcn_b200.train import DiffGraph, FlatParams, Trainer
 from oracle import cistgcn_oracle as O
 
@@ -29,7 +30,7 @@ def _log_parity(title, rows):
 
 
 def _reference_step(E, V, sd, x, tgt, train=True, input_grad=False, interp=True, dtype=torch.float32, device="cpu"):
-    ref = R.build(E, V, interpretable=interp, dropout=0.0).to(dtype)
+    ref = M.oracle_module(E, V, interp=interp).to(dtype)
     ref.load_state_dict(sd)
     ref = ref.to(device)
     ref.train(train)
@@ -152,21 +153,18 @@ def _compare(E, V, B, lib, device, interp=True, train=True, input_grad=False, dr
     return worst
 
 
-@pytest.mark.skipif(not R.available(), reason="reference module not available")
 def test_train_step_gradients_match_reference_autograd_emulated():
     import _emu
     worst = _compare(8, 22, 3, _emu.lib(), "cpu")
     print("worst relative gradient error", worst)
 
 
-@pytest.mark.skipif(not R.available(), reason="reference module not available")
 def test_eval_mode_input_gradient_matches_reference_emulated():
     import _emu
     _compare(8, 18, 2, _emu.lib(), "cpu", train=False, input_grad=True)
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not R.available(), reason="reference module not available")
 @pytest.mark.parametrize("E,V,B,interp", [(8, 22, 16, True), (32, 22, 24, True), (16, 18, 8, True), (8, 22, 6, False)])
 def test_train_step_gradients_match_reference_autograd_gpu(E, V, B, interp):
     from cistgcn_b200 import _cabi
@@ -174,14 +172,12 @@ def test_train_step_gradients_match_reference_autograd_gpu(E, V, B, interp):
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not R.available(), reason="reference module not available")
 def test_eval_mode_input_gradient_gpu():
     from cistgcn_b200 import _cabi
     _compare(32, 22, 8, _cabi.lib(), "cuda:0", train=False, input_grad=True)
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not R.available(), reason="reference module not available")
 def test_adam_steps_track_torch_optim_adam():
     """Three full steps (forward, loss, backward, fused Adam with L2-in-gradient weight decay) against the reference
     module + torch.optim.Adam (environment/utils.py:53-57): losses and parameters stay together."""
@@ -189,7 +185,7 @@ def test_adam_steps_track_torch_optim_adam():
     E, V, B = 16, 22, 32
     model0, sd, cfg = M.build(E, V, "W2")
     x, tgt = O.synth_inputs(B, cfg)
-    ref = R.build(E, V, dropout=0.0)
+    ref = M.oracle_module(E, V)
     ref.load_state_dict(sd)
     ref.train()
     LR = 1e-4          # Adam's update is ~lr * sign(g) at first: a small lr keeps the two fp32 trajectories comparable
@@ -219,7 +215,6 @@ def test_adam_steps_track_torch_optim_adam():
 
 
 @pytest.mark.gpu
-@pytest.mark.skipif(not R.available(), reason="reference module not available")
 def test_reference_style_training_loop_through_autograd():
     """environment/train.py:54-107 verbatim against the drop-in module: model.train(); outputs = model(inputs);
     loss = mpjpe(target, outputs[0]); optimizer.zero_grad(); loss.backward(); optimizer.step() with torch.optim.Adam."""
@@ -227,7 +222,7 @@ def test_reference_style_training_loop_through_autograd():
     E, V, B = 16, 22, 16
     model0, sd, cfg = M.build(E, V, "W2")
     x, tgt = O.synth_inputs(B, cfg)
-    ref = R.build(E, V, dropout=0.0)
+    ref = M.oracle_module(E, V)
     ref.load_state_dict(sd)
     ref.train()
     opt_ref = torch.optim.Adam(ref.parameters(), lr=1e-4, weight_decay=1e-4)
