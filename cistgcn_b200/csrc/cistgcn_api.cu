@@ -138,6 +138,10 @@ int launch_dstd_fused(const int32_t* desc, const float* weights, const float* in
   a.tap_w1 = taps ? taps->w1 : nullptr;
   a.tap_w2 = taps ? taps->w2 : nullptr;
   const int T = a.d[CB_T], V = a.d[CB_V], Ci = a.d[CB_CI], Co = a.d[CB_CO];
+  // 10-frame output blocks (output_n = 10) run on the three-stage path only: this kernel is not built for them
+  if (V == 10 && (T == 22 || T == 18))
+    return fail(-2, "DSTD-GC block: (T, V) = (%d, %d) (10-frame output block) has no fused kernel; "
+                    "CISTGCN_FLAG_DSTD_FUSED / CISTGCN_FLAG_DSTD_TC cannot run it", T, V);
   if (!a.d[CB_INTERP]) { a.tap_adj_s = nullptr; a.tap_adj_t = nullptr; }
   a.phase_clocks = g_phase_clocks;
   a.stamp_iter = g_stamp_iter;
@@ -164,7 +168,7 @@ int launch_dstd_fused(const int32_t* desc, const float* weights, const float* in
   CG_TRY_DSTD(18, 25)
 #undef CG_TRY_DSTD
   return fail(-2, "DSTD-GC block: (T, V) = (%d, %d) has no compiled kernel "
-                  "(built: (10,22), (10,18), (22,25), (18,25))", T, V);
+                  "(built: (10,22), (10,18), (22,25), (18,25), (22,10), (18,10))", T, V);
 }
 
 // ---- three-stage path (csrc/dstd_reduce.cuh -> dstd_adj.cuh -> dstd_mix.cuh)
@@ -179,7 +183,12 @@ struct SplitPlan {
 };
 
 bool shape_has_split_kernels(int T, int V) {
-  return (T == 10 && (V == 22 || V == 18)) || (V == 25 && (T == 22 || T == 18));
+  return (T == 10 && (V == 22 || V == 18)) || ((V == 25 || V == 10) && (T == 22 || T == 18));
+}
+
+// Output blocks whose stage 3 runs warp-per-sample (dstd_mix_narrow.cuh) by default
+bool shape_has_narrow_mix(int T, int V) {
+  return (V == 25 || V == 10) && (T == 22 || T == 18);
 }
 
 // Fills the three argument blocks' plans; false if the shape / widths are outside what the split kernels tile.
@@ -204,7 +213,7 @@ bool split_plan(const int32_t* desc, SplitPlan& sp, uint32_t flags = 0) {
   sp.mix_mma = false;
   sp.mix_narrow = false;
   // 3 -> 3 blocks (the output block): one warp per sample, adjacencies streamed from global memory
-  if (!(flags & CISTGCN_FLAG_DSTD_MIX_FFMA) && V == 25 && (T == 22 || T == 18) && cg::mix_narrow_plan<3>(sp.m, cap)) {
+  if (!(flags & CISTGCN_FLAG_DSTD_MIX_FFMA) && shape_has_narrow_mix(T, V) && cg::mix_narrow_plan<3>(sp.m, cap)) {
     sp.mix_narrow = true; sp.mix_nt = 32 * sp.m.nwarps; sp.mix_tm = 0;
   } else
   // tensor-core channel mixes: the input blocks (T = 10) from 16 channels up -- below that a 16-row MMA tile is mostly
@@ -243,6 +252,8 @@ bool use_split(const int32_t* desc, uint32_t flags, SplitPlan& sp) {
 int launch_mix_narrow_shape(int T, int V, const cg::MixArgs& m, void* stream) {
   if (T == 22 && V == 25) return cg::launch_mix_narrow_22_25(m, stream);
   if (T == 18 && V == 25) return cg::launch_mix_narrow_18_25(m, stream);
+  if (T == 22 && V == 10) return cg::launch_mix_narrow_22_10(m, stream);
+  if (T == 18 && V == 10) return cg::launch_mix_narrow_18_10(m, stream);
   return -1;
 }
 
@@ -289,8 +300,11 @@ int launch_dstd_split(SplitPlan& sp, const float* weights, const float* in, floa
   CG_SPLIT_SHAPE(10, 18)
   CG_SPLIT_SHAPE(22, 25)
   CG_SPLIT_SHAPE(18, 25)
+  CG_SPLIT_SHAPE(22, 10)
+  CG_SPLIT_SHAPE(18, 10)
 #undef CG_SPLIT_SHAPE
-  return fail(-2, "DSTD-GC block: (T, V) = (%d, %d) has no compiled kernel", T, V);
+  return fail(-2, "DSTD-GC block: (T, V) = (%d, %d) has no compiled kernel "
+                  "(built: (10,22), (10,18), (22,25), (18,25), (22,10), (18,10))", T, V);
 }
 
 // Scratch floats of one block for `batch` samples (0 when the block runs on the fused kernel).
@@ -318,13 +332,15 @@ int launch_dstd(const int32_t* desc, const float* weights, const float* in, floa
 }
 
 #ifndef CISTGCN_EMU
-// tcgen05 kernel (fpn_tc.cuh): 32-wide channel tiles, two 128-position tiles, weights packed with CF_TC_*
+// tcgen05 kernel (fpn_tc.cuh): 32-wide channel tiles, two 128-position tiles, weights packed with CF_TC_*.
+// A layer's K is its input channels padded to 16 (one k-step): 2 k-chunks for input_n <= 16 and output_n <= 16,
+// 4 for 16 < output_n <= 25.  The map's channels past output_n stay zero, so a 2-chunk layer reads only channels 0..15.
 bool fpn_tc_supported(const int32_t* fpn_descs, int n_fpn, const int32_t* tail_desc) {
   const int To = tail_desc[CT_TOUT], V = tail_desc[CT_V], Tin = tail_desc[CT_TIN];
   if (To > 25 || Tin > 16 || tail_desc[CT_F] != cg::FTC_F || (V != 22 && V != 18) || n_fpn > 4) return false;
   for (int l = 0; l < n_fpn; ++l) {
     const int32_t* f = fpn_descs + l * CF_COUNT;
-    if (f[CF_TC_KC] != (l == 0 ? 2 : 4) || f[CF_TC_W] <= 0 || f[CF_TC_PRM] <= 0) return false;
+    if (f[CF_TC_KC] != (f[CF_CIN] + 15) / 16 * 2 || f[CF_TC_W] <= 0 || f[CF_TC_PRM] <= 0) return false;
     if ((f[CF_RESID] != 0) != (l > 0)) return false;       // layer 0 reads the separate input buffer, no residual there
   }
   return true;

@@ -22,10 +22,14 @@ CG_DECL_SPLIT(10, 22)
 CG_DECL_SPLIT(10, 18)
 CG_DECL_SPLIT(22, 25)
 CG_DECL_SPLIT(18, 25)
+CG_DECL_SPLIT(22, 10)
+CG_DECL_SPLIT(18, 10)
 #undef CG_DECL_SPLIT
 int launch_mix_mma_10_22(const MixArgs& a, void* stream);
 int launch_mix_mma_10_18(const MixArgs& a, void* stream);
 int launch_mix_narrow_22_25(const MixArgs& a, void* stream);
 int launch_mix_narrow_18_25(const MixArgs& a, void* stream);
+int launch_mix_narrow_22_10(const MixArgs& a, void* stream);
+int launch_mix_narrow_18_10(const MixArgs& a, void* stream);
 
 }  // namespace cg

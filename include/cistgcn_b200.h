@@ -62,7 +62,7 @@ enum cistgcn_block_field {
   CB_CI = 0,      /* input channels */
   CB_CO,          /* output channels */
   CB_T,           /* length of the block's "time" axis  (10; V for the output block) */
-  CB_V,           /* length of the block's "joint" axis (V; 25 for the output block) */
+  CB_V,           /* length of the block's "joint" axis (V; output_n, 25 or 10, for the output block) */
   CB_CH,          /* Map2Adj inter channels = Ci/2            (CISTGCN.py:137) */
   CB_CG,          /* gate inter channels = max(Co/2,1)        (CISTGCN.py:321) */
   CB_HS,          /* SE hidden width = max(Co/reduction,1)    (SE.py:28-29)    */
@@ -118,7 +118,7 @@ enum cistgcn_block_field {
 /* ---- one FPN layer (CISTGCN.py:38-79) + the caller's PReLU / residual (:584-586) ------------ */
 enum cistgcn_fpn_field {
   CF_CIN = 0,     /* input channels (= frames): input_n for layer 0, output_n afterwards */
-  CF_COUT,        /* output_n (25) */
+  CF_COUT,        /* output_n (25 or 10) */
   CF_RESID,       /* 1: x6 = PReLU(FPN(x6)) + x6 (layers >= 1) */
   CF_W_D1, CF_W_D2, CF_W_D3,   /* block{1,2,3}.0 (+BN .1): [Cin][3][5 otiles][16] (kw-major, 5 outs, 1 pad) */
   CF_B_D1, CF_B_D2, CF_B_D3,   /* folded bias [Cout] */
