@@ -25,22 +25,13 @@ namespace {
 
 thread_local std::string g_err;
 
-int fail(int code, const char* fmt, ...) {
-  char buf[512];
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(buf, sizeof(buf), fmt, ap);
-  va_end(ap);
-  g_err = buf;
-  return code;
-}
-
 constexpr int kMaxSmemBytes = 227 * 1024;
 
 }  // namespace
 
 namespace cgt {
-// error sink of the training-op translation unit (train_ops.cu): same thread-local message as every other entry point
+// Records the message for cistgcn_last_error() and returns code: the error sink of every entry point, also those of
+// train_ops.cu, augment.cu and eval_metrics.cu
 int fail_train(int code, const char* fmt, ...) {
   char buf[512];
   va_list ap;
@@ -54,11 +45,13 @@ int fail_train(int code, const char* fmt, ...) {
 
 namespace {
 
+constexpr auto& fail = cgt::fail_train;
 using cg::sm_count;
 using cg::grid_for;
 
-int check_launch(const char* what) {
-  if (int e = cg::last_launch_error()) return fail(-4, "%s launch: %s", what, cg::launch_error_string(e));
+// e: what a launcher returned (a CUDA error code or 0)
+int check_launch(int e, const char* what) {
+  if (e) return fail(-4, "%s launch: %s", what, cg::launch_error_string(e));
   return 0;
 }
 
@@ -112,11 +105,6 @@ constexpr long long* g_phase_clocks = nullptr;
 constexpr int g_stamp_iter = 0;
 #endif
 
-int dstd_done(int e, const char* what) {
-  if (e) return fail(-4, "%s launch: %s", what, cg::launch_error_string(e));
-  return 0;
-}
-
 int check_block_desc(const int32_t* d) {
   const int Ci = d[CB_CI], Co = d[CB_CO];
   if (Ci < 2 || Co < 1) return fail(-2, "DSTD-GC block needs Ci >= 2 (got %d -> %d)", Ci, Co);
@@ -125,7 +113,18 @@ int check_block_desc(const int32_t* d) {
   return 0;
 }
 
+// one " (T,V)" per table line, for the "built:" list of an error message
+#define CG_SHAPE_NAME(T, V, ...) " (" #T "," #V ")"
+#define CG_JOINTS_NAME(V) " " #V
+
 // ---- round-1 fused kernel (one CTA per sample, csrc/dstd_block.cuh): E = 64 blocks and CISTGCN_FLAG_DSTD_FUSED
+template <int T, int V>
+int launch_fused_shape(const cg::DstdArgs& a, int nt, void* stream) {
+  if constexpr (cg::fused_shape(T, V)->tc)
+    if (nt == 512 && a.tc) return cg::launch_dstd_impl<T, V, 512, true>(a, stream);
+  return nt == 256 ? cg::launch_dstd_impl<T, V, 256>(a, stream) : cg::launch_dstd_impl<T, V, 512>(a, stream);
+}
+
 int launch_dstd_fused(const int32_t* desc, const float* weights, const float* in, float* out, long long batch,
                       const cistgcn_block_taps* taps, uint32_t flags, int in_bf16, int out_bf16, void* stream) {
   cg::DstdArgs a;
@@ -138,17 +137,17 @@ int launch_dstd_fused(const int32_t* desc, const float* weights, const float* in
   a.tap_w1 = taps ? taps->w1 : nullptr;
   a.tap_w2 = taps ? taps->w2 : nullptr;
   const int T = a.d[CB_T], V = a.d[CB_V], Ci = a.d[CB_CI], Co = a.d[CB_CO];
-  // 10-frame output blocks (output_n = 10) run on the three-stage path only: this kernel is not built for them
-  if (V == 10 && (T == 22 || T == 18))
-    return fail(-2, "DSTD-GC block: (T, V) = (%d, %d) (10-frame output block) has no fused kernel; "
-                    "CISTGCN_FLAG_DSTD_FUSED / CISTGCN_FLAG_DSTD_TC cannot run it", T, V);
+  // the 10-frame output blocks (output_n = 10) among others: they run on the three-stage path only
+  const cg::FusedShape* shape = cg::fused_shape(T, V);
+  if (!shape)
+    return fail(-2, "DSTD-GC block: (T, V) = (%d, %d) has no fused kernel (built:" CG_FUSED_SHAPES(CG_SHAPE_NAME) ")", T, V);
   if (!a.d[CB_INTERP]) { a.tap_adj_s = nullptr; a.tap_adj_t = nullptr; }
   a.phase_clocks = g_phase_clocks;
   a.stamp_iter = g_stamp_iter;
   // narrow blocks: 256 threads, two CTAs per SM (if the whole plan fits half an SM's shared memory);
   // wide blocks: 512 threads, one CTA per SM
   // (the tensor-core flag asks for the wide plan outright: only that instantiation carries the tcgen05 channel mixes)
-  const bool tc_ok = (flags & CISTGCN_FLAG_DSTD_TC) && T == 10 && (V == 22 || V == 18);   // shapes with a tensor-core instantiation
+  const bool tc_ok = (flags & CISTGCN_FLAG_DSTD_TC) && shape->tc;
   int nt = cg::DSTD_NT_NARROW;
   if (tc_ok || !cg::dstd_plan(a, nt, cg::DSTD_SMEM_NARROW_BYTES / 4)) {
     nt = cg::DSTD_NT_WIDE;
@@ -157,18 +156,12 @@ int launch_dstd_fused(const int32_t* desc, const float* weights, const float* in
                   (size_t)a.smem_floats * 4, kMaxSmemBytes);
   }
   ProfScope prof(KIND_DSTD, stream);
-  if (nt == 512 && a.tc)
-    return dstd_done(V == 22 ? cg::launch_dstd_10_22_512_tc(a, stream) : cg::launch_dstd_10_18_512_tc(a, stream), "dstd_block_kernel");
-#define CG_TRY_DSTD(TT, VV) \
-  if (T == TT && V == VV) \
-    return dstd_done(nt == 256 ? cg::launch_dstd_##TT##_##VV##_256(a, stream) : cg::launch_dstd_##TT##_##VV##_512(a, stream), "dstd_block_kernel");
-  CG_TRY_DSTD(10, 22)
-  CG_TRY_DSTD(10, 18)
-  CG_TRY_DSTD(22, 25)
-  CG_TRY_DSTD(18, 25)
-#undef CG_TRY_DSTD
-  return fail(-2, "DSTD-GC block: (T, V) = (%d, %d) has no compiled kernel "
-                  "(built: (10,22), (10,18), (22,25), (18,25), (22,10), (18,10))", T, V);
+  int e = 0;
+#define CG_FUSED_CASE(TT, VV, TC) \
+  if (T == TT && V == VV) e = launch_fused_shape<TT, VV>(a, nt, stream);
+  CG_FUSED_SHAPES(CG_FUSED_CASE)
+#undef CG_FUSED_CASE
+  return check_launch(e, "dstd_block_kernel");
 }
 
 // ---- three-stage path (csrc/dstd_reduce.cuh -> dstd_adj.cuh -> dstd_mix.cuh)
@@ -182,20 +175,12 @@ struct SplitPlan {
   size_t red_floats, wg_floats, adjs_floats, adjt_floats;     // scratch per sample
 };
 
-bool shape_has_split_kernels(int T, int V) {
-  return (T == 10 && (V == 22 || V == 18)) || ((V == 25 || V == 10) && (T == 22 || T == 18));
-}
-
-// Output blocks whose stage 3 runs warp-per-sample (dstd_mix_narrow.cuh) by default
-bool shape_has_narrow_mix(int T, int V) {
-  return (V == 25 || V == 10) && (T == 22 || T == 18);
-}
-
 // Fills the three argument blocks' plans; false if the shape / widths are outside what the split kernels tile.
 bool split_plan(const int32_t* desc, SplitPlan& sp, uint32_t flags = 0) {
   const int T = desc[CB_T], V = desc[CB_V], Co = desc[CB_CO], Ch = desc[CB_CH], Cg = desc[CB_CG];
   const bool interp = desc[CB_INTERP] != 0;
-  if (!shape_has_split_kernels(T, V)) return false;
+  const cg::SplitShape* shape = cg::split_shape(T, V);
+  if (!shape) return false;
   memcpy(sp.r.d, desc, sizeof(sp.r.d));
   memcpy(sp.j.d, desc, sizeof(sp.j.d));
   memcpy(sp.m.d, desc, sizeof(sp.m.d));
@@ -213,12 +198,12 @@ bool split_plan(const int32_t* desc, SplitPlan& sp, uint32_t flags = 0) {
   sp.mix_mma = false;
   sp.mix_narrow = false;
   // 3 -> 3 blocks (the output block): one warp per sample, adjacencies streamed from global memory
-  if (!(flags & CISTGCN_FLAG_DSTD_MIX_FFMA) && shape_has_narrow_mix(T, V) && cg::mix_narrow_plan<3>(sp.m, cap)) {
+  if (!(flags & CISTGCN_FLAG_DSTD_MIX_FFMA) && shape->mix_narrow && cg::mix_narrow_plan<3>(sp.m, cap)) {
     sp.mix_narrow = true; sp.mix_nt = 32 * sp.m.nwarps; sp.mix_tm = 0;
   } else
   // tensor-core channel mixes: the input blocks (T = 10) from 16 channels up -- below that a 16-row MMA tile is mostly
   // padding and the FFMA loops are already short
-  if (!(flags & CISTGCN_FLAG_DSTD_MIX_FFMA) && T == 10 && (desc[CB_CI] >= 16 || Co >= 16) &&
+  if (!(flags & CISTGCN_FLAG_DSTD_MIX_FFMA) && shape->mix_mma && (desc[CB_CI] >= 16 || Co >= 16) &&
       cg::mix_mma_plan(sp.m, cg::DSTD_SMEM_NARROW_BYTES / 4)) {
     sp.mix_mma = true; sp.mix_nt = 256; sp.mix_tm = 0;
   } else if (cg::mix_plan(sp.m, 256, cg::DSTD_SMEM_NARROW_BYTES / 4)) {
@@ -249,18 +234,28 @@ bool use_split(const int32_t* desc, uint32_t flags, SplitPlan& sp) {
   return split_plan(desc, sp, flags);
 }
 
-int launch_mix_narrow_shape(int T, int V, const cg::MixArgs& m, void* stream) {
-  if (T == 22 && V == 25) return cg::launch_mix_narrow_22_25(m, stream);
-  if (T == 18 && V == 25) return cg::launch_mix_narrow_18_25(m, stream);
-  if (T == 22 && V == 10) return cg::launch_mix_narrow_22_10(m, stream);
-  if (T == 18 && V == 10) return cg::launch_mix_narrow_18_10(m, stream);
-  return -1;
+int no_split_kernel(int T, int V) {
+  return fail(-2, "DSTD-GC block: (T, V) = (%d, %d) has no compiled kernel (built:" CG_SPLIT_SHAPES(CG_SHAPE_NAME) ")", T, V);
 }
 
-int launch_mix_mma_shape(int T, int V, const cg::MixArgs& m, void* stream) {
-  if (T == 10 && V == 22) return cg::launch_mix_mma_10_22(m, stream);
-  if (T == 10 && V == 18) return cg::launch_mix_mma_10_18(m, stream);
-  return -1;
+// The three stages of one table shape; stage 3 as split_plan chose it, among the variants the table line has
+template <int T, int V>
+int launch_split_shape(const SplitPlan& sp, void* stream) {
+  constexpr cg::SplitShape shape = *cg::split_shape(T, V);
+  int e;
+  { ProfScope prof(KIND_REDUCE, stream);
+    e = sp.ne == 1 ? cg::launch_reduce_impl<T, V, 1>(sp.r, stream) : cg::launch_reduce_impl<T, V, 2>(sp.r, stream); }
+  if (e) return check_launch(e, "dstd_reduce_kernel");
+  { ProfScope prof(KIND_ADJ, stream); e = cg::launch_adj_impl<T, V>(sp.j, stream); }
+  if (e) return check_launch(e, "dstd_adj_kernel");
+  ProfScope prof(KIND_MIX, stream);
+  if constexpr (shape.mix_narrow)
+    if (sp.mix_narrow) return check_launch(cg::launch_mix_narrow_impl<T, V, 3>(sp.m, stream), "dstd_mix_kernel");
+  if constexpr (shape.mix_mma)
+    if (sp.mix_mma) return check_launch(cg::launch_mix_mma_impl<T, V>(sp.m, stream), "dstd_mix_kernel");
+  e = sp.mix_nt == 512 ? cg::launch_mix_impl<T, V, 512, 8>(sp.m, stream)
+      : sp.mix_tm == 8 ? cg::launch_mix_impl<T, V, 256, 8>(sp.m, stream) : cg::launch_mix_impl<T, V, 256, 4>(sp.m, stream);
+  return check_launch(e, "dstd_mix_kernel");
 }
 
 int launch_dstd_split(SplitPlan& sp, const float* weights, const float* in, float* out, long long batch,
@@ -281,30 +276,11 @@ int launch_dstd_split(SplitPlan& sp, const float* weights, const float* in, floa
   sp.j.adj_s = adj_s; sp.j.adj_t = adj_t; sp.j.batch = (int)batch;
   sp.j.tap_w1 = taps ? taps->w1 : nullptr; sp.j.tap_w2 = taps ? taps->w2 : nullptr;
   sp.m.w = weights; sp.m.in = in; sp.m.out = out; sp.m.wg = wg; sp.m.adj_s = adj_s; sp.m.adj_t = adj_t; sp.m.batch = (int)batch;
-  int e = -1;
-#define CG_SPLIT_SHAPE(TT, VV) \
-  if (T == TT && V == VV) { \
-    { ProfScope prof(KIND_REDUCE, stream); \
-      e = sp.ne == 1 ? cg::launch_reduce_##TT##_##VV##_1(sp.r, stream) : cg::launch_reduce_##TT##_##VV##_2(sp.r, stream); } \
-    if (e) return dstd_done(e, "dstd_reduce_kernel"); \
-    { ProfScope prof(KIND_ADJ, stream); e = cg::launch_adj_##TT##_##VV(sp.j, stream); } \
-    if (e) return dstd_done(e, "dstd_adj_kernel"); \
-    { ProfScope prof(KIND_MIX, stream); \
-      e = sp.mix_narrow ? launch_mix_narrow_shape(TT, VV, sp.m, stream) \
-          : sp.mix_mma ? launch_mix_mma_shape(TT, VV, sp.m, stream) \
-          : sp.mix_nt == 512 ? cg::launch_mix_##TT##_##VV##_512_8(sp.m, stream) \
-          : (sp.mix_tm == 8 ? cg::launch_mix_##TT##_##VV##_256_8(sp.m, stream) : cg::launch_mix_##TT##_##VV##_256_4(sp.m, stream)); } \
-    return dstd_done(e, "dstd_mix_kernel"); \
-  }
-  CG_SPLIT_SHAPE(10, 22)
-  CG_SPLIT_SHAPE(10, 18)
-  CG_SPLIT_SHAPE(22, 25)
-  CG_SPLIT_SHAPE(18, 25)
-  CG_SPLIT_SHAPE(22, 10)
-  CG_SPLIT_SHAPE(18, 10)
-#undef CG_SPLIT_SHAPE
-  return fail(-2, "DSTD-GC block: (T, V) = (%d, %d) has no compiled kernel "
-                  "(built: (10,22), (10,18), (22,25), (18,25), (22,10), (18,10))", T, V);
+#define CG_SPLIT_CASE(TT, VV, MMA, NARROW) \
+  if (T == TT && V == VV) return launch_split_shape<TT, VV>(sp, stream);
+  CG_SPLIT_SHAPES(CG_SPLIT_CASE)
+#undef CG_SPLIT_CASE
+  return no_split_kernel(T, V);
 }
 
 // Scratch floats of one block for `batch` samples (0 when the block runs on the fused kernel).
@@ -328,6 +304,9 @@ int launch_dstd(const int32_t* desc, const float* weights, const float* in, floa
       return fail(-1, "DSTD-GC block: scratch too small (%zu floats given, %zu needed)", scratch_floats, need);
     return launch_dstd_split(sp, weights, in, out, batch, taps, scratch, in_bf16, out_bf16, stream);
   }
+  // a shape neither path is built for: name the shapes of the default (three-stage) path
+  if (!(flags & (CISTGCN_FLAG_DSTD_FUSED | CISTGCN_FLAG_DSTD_TC)) && !cg::split_shape(desc[CB_T], desc[CB_V]))
+    return no_split_kernel(desc[CB_T], desc[CB_V]);
   return launch_dstd_fused(desc, weights, in, out, batch, taps, flags, in_bf16, out_bf16, stream);
 }
 
@@ -337,7 +316,7 @@ int launch_dstd(const int32_t* desc, const float* weights, const float* in, floa
 // 4 for 16 < output_n <= 25.  The map's channels past output_n stay zero, so a 2-chunk layer reads only channels 0..15.
 bool fpn_tc_supported(const int32_t* fpn_descs, int n_fpn, const int32_t* tail_desc) {
   const int To = tail_desc[CT_TOUT], V = tail_desc[CT_V], Tin = tail_desc[CT_TIN];
-  if (To > 25 || Tin > 16 || tail_desc[CT_F] != cg::FTC_F || (V != 22 && V != 18) || n_fpn > 4) return false;
+  if (To > 25 || Tin > 16 || tail_desc[CT_F] != cg::FTC_F || !cg::fpn_joints_built(V) || n_fpn > 4) return false;
   for (int l = 0; l < n_fpn; ++l) {
     const int32_t* f = fpn_descs + l * CF_COUNT;
     if (f[CF_TC_KC] != (f[CF_CIN] + 15) / 16 * 2 || f[CF_TC_W] <= 0 || f[CF_TC_PRM] <= 0) return false;
@@ -353,14 +332,13 @@ int launch_fpn_tc(const int32_t* fpn_descs, int n_fpn, const int32_t* tail_desc,
   memcpy(a.t, tail_desc, sizeof(a.t));
   a.n_layers = n_fpn; a.w = weights; a.in = in; a.x7 = x7; a.batch = (int)batch;
   a.dbg = g_phase_clocks;     // nullptr outside -DCISTGCN_PROFILE builds
-  int e;
-  {
-    ProfScope prof(KIND_FPN, stream);
-    if (bf16) e = a.t[CT_V] == 22 ? cg::launch_fpn_tc_22_bf16(a, stream) : cg::launch_fpn_tc_18_bf16(a, stream);
-    else e = a.t[CT_V] == 22 ? cg::launch_fpn_tc_22(a, stream) : cg::launch_fpn_tc_18(a, stream);
-  }
-  if (e) return fail(-4, "fpn_tc_kernel launch: %s", cg::launch_error_string(e));
-  return 0;
+  ProfScope prof(KIND_FPN, stream);
+  int e = 0;
+#define CG_FPN_TC_CASE(VV) \
+  if (a.t[CT_V] == VV) e = bf16 ? cg::launch_fpn_tc_impl<VV, true>(a, stream) : cg::launch_fpn_tc_impl<VV, false>(a, stream);
+  CG_FPN_JOINTS(CG_FPN_TC_CASE)
+#undef CG_FPN_TC_CASE
+  return check_launch(e, "fpn_tc_kernel");
 }
 #endif
 
@@ -400,15 +378,15 @@ int launch_fpn(const int32_t* fpn_descs, int n_fpn, const int32_t* tail_desc, co
   cg::fpn_plan(a);
   const size_t smem = (size_t)a.smem_floats * sizeof(float);
   if (smem > (size_t)kMaxSmemBytes) return fail(-2, "FPN chain needs %zu B of shared memory", smem);
-  int e;
-  {
-    ProfScope prof(KIND_FPN, stream);
-    if (V == 22) e = cg::launch_fpn_22(a, stream);
-    else if (V == 18) e = cg::launch_fpn_18(a, stream);
-    else return fail(-2, "FPN chain: joints = %d has no compiled kernel (built: 22, 18)", V);
-  }
-  if (e) return fail(-4, "fpn_chain_kernel launch: %s", cg::launch_error_string(e));
-  return 0;
+  if (!cg::fpn_joints_built(V))
+    return fail(-2, "FPN chain: joints = %d has no compiled kernel (built:" CG_FPN_JOINTS(CG_JOINTS_NAME) ")", V);
+  ProfScope prof(KIND_FPN, stream);
+  int e = 0;
+#define CG_FPN_CASE(VV) \
+  if (V == VV) e = cg::launch_fpn_impl<VV>(a, stream);
+  CG_FPN_JOINTS(CG_FPN_CASE)
+#undef CG_FPN_CASE
+  return check_launch(e, "fpn_chain_kernel");
 }
 
 int launch_tail(const int32_t* tail_desc, const float* weights, const float* x, const float* x7, const float* x8,
@@ -436,7 +414,7 @@ int launch_tail(const int32_t* tail_desc, const float* weights, const float* x, 
   const int grid = grid_for(batch, per_sm);
   ProfScope prof(KIND_TAIL, stream);
   CG_LAUNCH(kfn, grid, cg::TAIL_NT, smem, stream, a);
-  return check_launch("tail_kernel");
+  return check_launch(cg::last_launch_error(), "tail_kernel");
 }
 
 struct PlanView {
@@ -678,7 +656,7 @@ int cistgcn_mpjpe_f32(const float* pred, const float* target, int64_t batch, int
   auto kfn = cg::mpjpe_kernel;
   ProfScope prof(KIND_MPJPE, stream);
   CG_LAUNCH(kfn, (int)(blocks < cap ? blocks : cap), 256, 0, stream, a);
-  return check_launch("mpjpe_kernel");
+  return check_launch(cg::last_launch_error(), "mpjpe_kernel");
 }
 
 }  // extern "C"

@@ -462,7 +462,7 @@ __global__ void __launch_bounds__(32 * (MMA ? ADJ_MMA_MAX_WARPS : ADJ_MAX_WARPS)
 }
 
 template <int T, int V>
-inline int launch_adj_impl(const AdjArgs& a, void* stream) {
+int launch_adj_impl(const AdjArgs& a, void* stream) {
   if (a.mma) return launch_warp_per_sample(dstd_adj_kernel<T, V, true>, a, stream);
   return launch_warp_per_sample(dstd_adj_kernel<T, V, false>, a, stream);
 }

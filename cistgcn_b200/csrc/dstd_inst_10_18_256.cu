@@ -1,5 +1,3 @@
 // Explicit instantiation of the fused DSTD-GC kernel for (T, V) = (10, 18), 256 threads per CTA.
 #include "dstd_launch.h"
-namespace cg {
-int launch_dstd_10_18_256(const DstdArgs& a, void* stream) { return launch_dstd_impl<10, 18, 256>(a, stream); }
-}  // namespace cg
+template int cg::launch_dstd_impl<10, 18, 256>(const cg::DstdArgs&, void*);

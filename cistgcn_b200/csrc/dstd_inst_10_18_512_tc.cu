@@ -1,9 +1,3 @@
 // Explicit instantiation of the fused DSTD-GC kernel for T = 10, V = 18, 512 threads, tensor-core channel mixes.
 #include "dstd_launch.h"
-namespace cg {
-#ifndef CISTGCN_EMU
-int launch_dstd_10_18_512_tc(const DstdArgs& a, void* stream) { return launch_dstd_impl<10, 18, 512, true>(a, stream); }
-#else
-int launch_dstd_10_18_512_tc(const DstdArgs& a, void* stream) { return launch_dstd_impl<10, 18, 512, false>(a, stream); }
-#endif
-}  // namespace cg
+template int cg::launch_dstd_impl<10, 18, 512, true>(const cg::DstdArgs&, void*);

@@ -1,5 +1,3 @@
 // Explicit instantiation of the fused DSTD-GC kernel for (T, V) = (10, 22), 256 threads per CTA.
 #include "dstd_launch.h"
-namespace cg {
-int launch_dstd_10_22_256(const DstdArgs& a, void* stream) { return launch_dstd_impl<10, 22, 256>(a, stream); }
-}  // namespace cg
+template int cg::launch_dstd_impl<10, 22, 256>(const cg::DstdArgs&, void*);

@@ -1,5 +1,3 @@
 // Explicit instantiation of the fused DSTD-GC kernel for (T, V) = (10, 22), 512 threads per CTA.
 #include "dstd_launch.h"
-namespace cg {
-int launch_dstd_10_22_512(const DstdArgs& a, void* stream) { return launch_dstd_impl<10, 22, 512>(a, stream); }
-}  // namespace cg
+template int cg::launch_dstd_impl<10, 22, 512>(const cg::DstdArgs&, void*);

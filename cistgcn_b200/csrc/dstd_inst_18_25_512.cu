@@ -1,5 +1,3 @@
 // Explicit instantiation of the fused DSTD-GC kernel for (T, V) = (18, 25), 512 threads per CTA.
 #include "dstd_launch.h"
-namespace cg {
-int launch_dstd_18_25_512(const DstdArgs& a, void* stream) { return launch_dstd_impl<18, 25, 512>(a, stream); }
-}  // namespace cg
+template int cg::launch_dstd_impl<18, 25, 512>(const cg::DstdArgs&, void*);

@@ -357,7 +357,7 @@ __global__ void __launch_bounds__(NT, NT <= 256 ? 2 : 1) dstd_mix_kernel(const M
 }
 
 template <int T, int V, int NT, int TM>
-inline int launch_mix_impl(const MixArgs& a, void* stream) {
+int launch_mix_impl(const MixArgs& a, void* stream) {
   auto kfn = dstd_mix_kernel<T, V, NT, TM>;
   const size_t smem = (size_t)a.smem_floats * sizeof(float);
   int err = 0;

@@ -1,5 +1,3 @@
 // Explicit instantiation: mix stage of the three-stage DSTD-GC path, (T, V) = (10, 18), 512 threads, TM = 8.
 #include "dstd_mix.cuh"
-namespace cg {
-int launch_mix_10_18_512_8(const MixArgs& a, void* stream) { return launch_mix_impl<10, 18, 512, 8>(a, stream); }
-}  // namespace cg
+template int cg::launch_mix_impl<10, 18, 512, 8>(const cg::MixArgs&, void*);

@@ -1,5 +1,3 @@
 // Explicit instantiation: mix stage of the three-stage DSTD-GC path, (T, V) = (18, 25), 256 threads, TM = 4.
 #include "dstd_mix.cuh"
-namespace cg {
-int launch_mix_18_25_256_4(const MixArgs& a, void* stream) { return launch_mix_impl<18, 25, 256, 4>(a, stream); }
-}  // namespace cg
+template int cg::launch_mix_impl<18, 25, 256, 4>(const cg::MixArgs&, void*);

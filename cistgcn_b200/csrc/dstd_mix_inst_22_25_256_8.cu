@@ -1,5 +1,3 @@
 // Explicit instantiation: mix stage of the three-stage DSTD-GC path, (T, V) = (22, 25), 256 threads, TM = 8.
 #include "dstd_mix.cuh"
-namespace cg {
-int launch_mix_22_25_256_8(const MixArgs& a, void* stream) { return launch_mix_impl<22, 25, 256, 8>(a, stream); }
-}  // namespace cg
+template int cg::launch_mix_impl<22, 25, 256, 8>(const cg::MixArgs&, void*);

@@ -510,7 +510,7 @@ inline int launch_mix_mma_mt(const MixArgs& a, void* stream) {
   return last_launch_error();
 }
 template <int T, int V>
-inline int launch_mix_mma_impl(const MixArgs& a, void* stream) {
+int launch_mix_mma_impl(const MixArgs& a, void* stream) {
   return mma_mt(a.d[CB_CO]) == 1 ? launch_mix_mma_mt<T, V, 1>(a, stream) : launch_mix_mma_mt<T, V, 2>(a, stream);
 }
 

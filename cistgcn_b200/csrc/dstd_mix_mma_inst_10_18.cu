@@ -1,5 +1,3 @@
 // Explicit instantiation: tensor-core (3xTF32 mma.sync) mix stage of the three-stage DSTD-GC path, (T, V) = (10, 18).
 #include "dstd_mix_mma.cuh"
-namespace cg {
-int launch_mix_mma_10_18(const MixArgs& a, void* stream) { return launch_mix_mma_impl<10, 18>(a, stream); }
-}  // namespace cg
+template int cg::launch_mix_mma_impl<10, 18>(const cg::MixArgs&, void*);

@@ -260,7 +260,7 @@ __global__ void __launch_bounds__(32 * MIXN_MAX_WARPS, 1) dstd_mix_narrow_kernel
 }
 
 template <int T, int V, int C>
-inline int launch_mix_narrow_impl(const MixArgs& a, void* stream) {
+int launch_mix_narrow_impl(const MixArgs& a, void* stream) {
   return launch_warp_per_sample(dstd_mix_narrow_kernel<T, V, C>, a, stream);
 }
 

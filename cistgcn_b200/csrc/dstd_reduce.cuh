@@ -666,7 +666,7 @@ __global__ void __launch_bounds__(32 * RED_MAX_WARPS, 1) dstd_reduce_kernel(cons
 }
 
 template <int T, int V, int NE>
-inline int launch_reduce_impl(const ReduceArgs& a, void* stream) {
+int launch_reduce_impl(const ReduceArgs& a, void* stream) {
   if constexpr (T == 10) {
     if (a.mma) return launch_warp_per_sample(dstd_reduce_kernel<T, V, NE, true>, a, stream);
   }

@@ -1,8 +1,6 @@
 // Explicit instantiations: reduce + adjacency stages of the three-stage DSTD-GC path for (T, V) = (10, 18).
 #include "dstd_adj.cuh"
 #include "dstd_reduce.cuh"
-namespace cg {
-int launch_reduce_10_18_1(const ReduceArgs& a, void* stream) { return launch_reduce_impl<10, 18, 1>(a, stream); }
-int launch_reduce_10_18_2(const ReduceArgs& a, void* stream) { return launch_reduce_impl<10, 18, 2>(a, stream); }
-int launch_adj_10_18(const AdjArgs& a, void* stream) { return launch_adj_impl<10, 18>(a, stream); }
-}  // namespace cg
+template int cg::launch_reduce_impl<10, 18, 1>(const cg::ReduceArgs&, void*);
+template int cg::launch_reduce_impl<10, 18, 2>(const cg::ReduceArgs&, void*);
+template int cg::launch_adj_impl<10, 18>(const cg::AdjArgs&, void*);

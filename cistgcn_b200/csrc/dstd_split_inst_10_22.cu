@@ -1,8 +1,6 @@
 // Explicit instantiations: reduce + adjacency stages of the three-stage DSTD-GC path for (T, V) = (10, 22).
 #include "dstd_adj.cuh"
 #include "dstd_reduce.cuh"
-namespace cg {
-int launch_reduce_10_22_1(const ReduceArgs& a, void* stream) { return launch_reduce_impl<10, 22, 1>(a, stream); }
-int launch_reduce_10_22_2(const ReduceArgs& a, void* stream) { return launch_reduce_impl<10, 22, 2>(a, stream); }
-int launch_adj_10_22(const AdjArgs& a, void* stream) { return launch_adj_impl<10, 22>(a, stream); }
-}  // namespace cg
+template int cg::launch_reduce_impl<10, 22, 1>(const cg::ReduceArgs&, void*);
+template int cg::launch_reduce_impl<10, 22, 2>(const cg::ReduceArgs&, void*);
+template int cg::launch_adj_impl<10, 22>(const cg::AdjArgs&, void*);

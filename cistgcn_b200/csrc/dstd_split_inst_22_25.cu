@@ -2,9 +2,7 @@
 #include "dstd_adj.cuh"
 #include "dstd_mix_narrow.cuh"
 #include "dstd_reduce.cuh"
-namespace cg {
-int launch_reduce_22_25_1(const ReduceArgs& a, void* stream) { return launch_reduce_impl<22, 25, 1>(a, stream); }
-int launch_reduce_22_25_2(const ReduceArgs& a, void* stream) { return launch_reduce_impl<22, 25, 2>(a, stream); }
-int launch_adj_22_25(const AdjArgs& a, void* stream) { return launch_adj_impl<22, 25>(a, stream); }
-int launch_mix_narrow_22_25(const MixArgs& a, void* stream) { return launch_mix_narrow_impl<22, 25, 3>(a, stream); }
-}  // namespace cg
+template int cg::launch_reduce_impl<22, 25, 1>(const cg::ReduceArgs&, void*);
+template int cg::launch_reduce_impl<22, 25, 2>(const cg::ReduceArgs&, void*);
+template int cg::launch_adj_impl<22, 25>(const cg::AdjArgs&, void*);
+template int cg::launch_mix_narrow_impl<22, 25, 3>(const cg::MixArgs&, void*);

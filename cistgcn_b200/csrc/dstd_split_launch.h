@@ -1,6 +1,7 @@
-// Launchers of the three-stage DSTD-GC path (dstd_reduce.cuh, dstd_adj.cuh, dstd_mix.cuh), one translation unit per
-// instantiation group so that nvcc compiles them in parallel (dstd_split_inst_*.cu, dstd_mix_inst_*.cu).
-// Return 0 or a CUDA error code.
+// Launchers of the three-stage DSTD-GC path (dstd_reduce.cuh, dstd_adj.cuh, dstd_mix*.cuh).  Each table shape of
+// kernel_shapes.h is instantiated in its own translation units (dstd_split_inst_*.cu, dstd_mix_inst_*.cu,
+// dstd_mix_mma_inst_*.cu) so that nvcc compiles them in parallel; the declarations below keep every other unit from
+// instantiating them again.  Launchers return 0 or a CUDA error code.
 #pragma once
 #include "dstd_adj.cuh"
 #include "dstd_mix.cuh"
@@ -8,28 +9,20 @@
 #include "dstd_mix_narrow.cuh"
 #include "dstd_reduce.cuh"
 #include "host_util.h"
+#include "kernel_shapes.h"
 
 namespace cg {
 
-#define CG_DECL_SPLIT(T, V) \
-  int launch_reduce_##T##_##V##_1(const ReduceArgs& a, void* stream); \
-  int launch_reduce_##T##_##V##_2(const ReduceArgs& a, void* stream); \
-  int launch_adj_##T##_##V(const AdjArgs& a, void* stream); \
-  int launch_mix_##T##_##V##_256_4(const MixArgs& a, void* stream); \
-  int launch_mix_##T##_##V##_256_8(const MixArgs& a, void* stream); \
-  int launch_mix_##T##_##V##_512_8(const MixArgs& a, void* stream);
-CG_DECL_SPLIT(10, 22)
-CG_DECL_SPLIT(10, 18)
-CG_DECL_SPLIT(22, 25)
-CG_DECL_SPLIT(18, 25)
-CG_DECL_SPLIT(22, 10)
-CG_DECL_SPLIT(18, 10)
-#undef CG_DECL_SPLIT
-int launch_mix_mma_10_22(const MixArgs& a, void* stream);
-int launch_mix_mma_10_18(const MixArgs& a, void* stream);
-int launch_mix_narrow_22_25(const MixArgs& a, void* stream);
-int launch_mix_narrow_18_25(const MixArgs& a, void* stream);
-int launch_mix_narrow_22_10(const MixArgs& a, void* stream);
-int launch_mix_narrow_18_10(const MixArgs& a, void* stream);
+#define CG_EXTERN_SPLIT(T, V, MMA, NARROW)                                                      \
+  extern template int launch_reduce_impl<T, V, 1>(const ReduceArgs&, void*);                     \
+  extern template int launch_reduce_impl<T, V, 2>(const ReduceArgs&, void*);                     \
+  extern template int launch_adj_impl<T, V>(const AdjArgs&, void*);                               \
+  extern template int launch_mix_impl<T, V, 256, 4>(const MixArgs&, void*);                       \
+  extern template int launch_mix_impl<T, V, 256, 8>(const MixArgs&, void*);                       \
+  extern template int launch_mix_impl<T, V, 512, 8>(const MixArgs&, void*);                       \
+  CG_IF_##MMA(extern template int launch_mix_mma_impl<T, V>(const MixArgs&, void*);)              \
+  CG_IF_##NARROW(extern template int launch_mix_narrow_impl<T, V, 3>(const MixArgs&, void*);)
+CG_SPLIT_SHAPES(CG_EXTERN_SPLIT)
+#undef CG_EXTERN_SPLIT
 
 }  // namespace cg

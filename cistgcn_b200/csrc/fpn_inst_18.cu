@@ -1,5 +1,3 @@
 // Explicit instantiation of the FPN-chain kernel for V = 18 joints.
 #include "fpn_launch.h"
-namespace cg {
-int launch_fpn_18(const FpnArgs& a, void* stream) { return launch_fpn_impl<18>(a, stream); }
-}  // namespace cg
+template int cg::launch_fpn_impl<18>(const cg::FpnArgs&, void*);

@@ -1,5 +1,3 @@
 // Explicit instantiation of the FPN-chain kernel for V = 22 joints.
 #include "fpn_launch.h"
-namespace cg {
-int launch_fpn_22(const FpnArgs& a, void* stream) { return launch_fpn_impl<22>(a, stream); }
-}  // namespace cg
+template int cg::launch_fpn_impl<22>(const cg::FpnArgs&, void*);

@@ -1,7 +1,5 @@
 // Explicit instantiation of the tensor-core FPN kernel for V = 18 joints.
 #include "fpn_tc_launch.h"
 #ifndef CISTGCN_EMU
-namespace cg {
-int launch_fpn_tc_18(const FpnTcArgs& a, void* stream) { return launch_fpn_tc_impl<18>(a, stream); }
-}  // namespace cg
+template int cg::launch_fpn_tc_impl<18>(const cg::FpnTcArgs&, void*);
 #endif

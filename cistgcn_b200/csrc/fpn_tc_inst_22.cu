@@ -1,7 +1,5 @@
 // Explicit instantiation of the tensor-core FPN kernel for V = 22 joints.
 #include "fpn_tc_launch.h"
 #ifndef CISTGCN_EMU
-namespace cg {
-int launch_fpn_tc_22(const FpnTcArgs& a, void* stream) { return launch_fpn_tc_impl<22>(a, stream); }
-}  // namespace cg
+template int cg::launch_fpn_tc_impl<22>(const cg::FpnTcArgs&, void*);
 #endif

@@ -1,7 +1,5 @@
 // Explicit instantiation of the tensor-core FPN kernel for V = 22 joints, single-term bf16 operands.
 #include "fpn_tc_launch.h"
 #ifndef CISTGCN_EMU
-namespace cg {
-int launch_fpn_tc_22_bf16(const FpnTcArgs& a, void* stream) { return launch_fpn_tc_impl<22, true>(a, stream); }
-}  // namespace cg
+template int cg::launch_fpn_tc_impl<22, true>(const cg::FpnTcArgs&, void*);
 #endif
