@@ -64,6 +64,13 @@ def bind(path: str) -> ctypes.CDLL:
                                       ctypes.c_int64, ctypes.POINTER(Taps), _p]
     L.cistgcn_forward_bf16.restype = ctypes.c_int
     L.cistgcn_forward_bf16.argtypes = L.cistgcn_forward_f32.argtypes
+    L.cistgcn_rollout_workspace_bytes.restype = ctypes.c_size_t
+    L.cistgcn_rollout_workspace_bytes.argtypes = [_i32p, ctypes.c_int64]
+    L.cistgcn_rollout_f32.restype = ctypes.c_int
+    L.cistgcn_rollout_f32.argtypes = [_i32p, ctypes.c_int32, _p, _p, ctypes.c_int32, _p, _p, _p, _p, ctypes.c_size_t,
+                                      ctypes.c_int64, _p]
+    L.cistgcn_rollout_bf16.restype = ctypes.c_int
+    L.cistgcn_rollout_bf16.argtypes = L.cistgcn_rollout_f32.argtypes
     L.cistgcn_dstd_block_f32.restype = ctypes.c_int
     L.cistgcn_dstd_block_f32.argtypes = [_i32p, _p, _p, _p, ctypes.c_int64, ctypes.POINTER(BlockTaps), _p, ctypes.c_size_t,
                                          ctypes.c_uint32, _p]

@@ -21,6 +21,12 @@
 #define CISTGCN_MAX_CHUNK 32768
 #endif
 
+namespace cg {
+// csrc/rollout.cu: moves one rollout step's prediction into the output and the next input window; 0 or a CUDA error
+int launch_rollout_step(const float* pred, float* out, float* window, const float* target, double* frame_sums,
+                        long long n, int t0, int nf, int H, int Tin, int To, int V, void* stream);
+}  // namespace cg
+
 namespace {
 
 thread_local std::string g_err;
@@ -528,6 +534,69 @@ size_t cistgcn_workspace_bytes(const int32_t* plan, int64_t batch) {
   return (2 * act + 2 * xo + scratch) * sizeof(float) + 256;
 }
 
+// The forward's per-chunk regions inside a caller's workspace (layout above); `end` is the first float past them
+struct ChunkWorkspace {
+  float *act0, *act1, *x7, *x8, *scratch, *end;
+  size_t scratch_floats;
+};
+
+static ChunkWorkspace chunk_workspace(const PlanView& pv, const int32_t* plan, long long chunk_max, void* workspace) {
+  const size_t act = align64f((size_t)chunk_max * act_floats_per_sample(plan));
+  const size_t xo = align64f((size_t)chunk_max * plan[CP_TOUT] * plan[CP_V] * 3);
+  ChunkWorkspace w;
+  w.act0 = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
+  w.act1 = w.act0 + act;
+  w.x7 = w.act1 + act;
+  w.x8 = w.x7 + xo;
+  w.scratch = w.x8 + xo;
+  w.scratch_floats = align64f(plan_scratch_floats(pv, (uint32_t)plan[CP_FLAGS], chunk_max));
+  w.end = w.scratch + w.scratch_floats;
+  return w;
+}
+
+// The whole model on one chunk of n samples: x (n, Tin, V, 3) -> pred (n, Tout, V, 3) (+ MPJPE sums against target);
+// s = the chunk's first sample in the taps
+static int forward_chunk(const PlanView& pv, const float* weights, const float* x, float* pred, const float* target,
+                         double* frame_sums, long long n, const cistgcn_taps* taps, long long s, const ChunkWorkspace& w,
+                         uint32_t flags, void* stream, bool act_bf16) {
+  auto block_taps = [&](const cistgcn_block_taps& src, const int32_t* bd) {
+    cistgcn_block_taps bt = {nullptr, nullptr, nullptr, nullptr};
+    const size_t tv = (size_t)bd[CB_T] * bd[CB_V];
+    bt.adj_s = src.adj_s ? src.adj_s + (size_t)s * tv * bd[CB_T] : nullptr;
+    bt.adj_t = src.adj_t ? src.adj_t + (size_t)s * tv * bd[CB_V] : nullptr;
+    bt.w1 = src.w1 ? src.w1 + (size_t)s * bd[CB_CO] : nullptr;
+    bt.w2 = src.w2 ? src.w2 + (size_t)s * bd[CB_CO] : nullptr;
+    return bt;
+  };
+  const float* cur = x;
+  float* bufs[2] = {w.act0, w.act1};
+  int flip = 0;
+  for (int i = 0; i < pv.n_in; ++i) {
+    const int32_t* bd = pv.in_blocks + i * CB_COUNT;
+    cistgcn_block_taps bt = {nullptr, nullptr, nullptr, nullptr};
+    if (taps) bt = block_taps(taps->in_blocks[i], bd);
+    float* dst = bufs[flip];
+    // bf16 forward: every inter-block activation of the input stack (and the FPN's input) is stored as bf16
+    if (int rc = launch_dstd(bd, weights, cur, dst, n, taps ? &bt : nullptr, w.scratch, w.scratch_floats, flags, stream,
+                             act_bf16 && i > 0, act_bf16))
+      return rc;
+    cur = dst;
+    flip ^= 1;
+  }
+  if (int rc = launch_fpn(pv.fpn, pv.n_fpn, pv.tail, weights, cur, w.x7, n, flags, stream, act_bf16)) return rc;
+  cur = w.x7;
+  for (int i = 0; i < pv.n_out; ++i) {
+    const int32_t* bd = pv.out_blocks + i * CB_COUNT;
+    cistgcn_block_taps bt = {nullptr, nullptr, nullptr, nullptr};
+    if (taps) bt = block_taps(taps->out_blocks[i], bd);
+    float* dst = (i == pv.n_out - 1) ? w.x8 : bufs[flip];
+    if (int rc = launch_dstd(bd, weights, cur, dst, n, taps ? &bt : nullptr, w.scratch, w.scratch_floats, flags, stream)) return rc;
+    cur = dst;
+    flip ^= 1;
+  }
+  return launch_tail(pv.tail, weights, x, w.x7, w.x8, pred, target, frame_sums, n, taps, s, stream);
+}
+
 static int forward_impl(const int32_t* plan, int32_t plan_len, const float* weights, const float* x, float* pred,
                         const float* target, double* frame_sums, void* workspace, size_t workspace_bytes,
                         int64_t batch, const cistgcn_taps* taps, void* stream, bool act_bf16) {
@@ -541,55 +610,12 @@ static int forward_impl(const int32_t* plan, int32_t plan_len, const float* weig
   const uint32_t flags = (uint32_t)plan[CP_FLAGS];
   const int T = plan[CP_TIN], To = plan[CP_TOUT], V = plan[CP_V];
   const long long chunk_max = batch < CISTGCN_MAX_CHUNK ? batch : CISTGCN_MAX_CHUNK;
-  const size_t act = align64f((size_t)chunk_max * act_floats_per_sample(plan));
-  const size_t xo = align64f((size_t)chunk_max * To * V * 3);
-  float* ws = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-  float* act0 = ws;
-  float* act1 = act0 + act;
-  float* x7 = act1 + act;
-  float* x8 = x7 + xo;
-  float* scratch = x8 + xo;
-  const size_t scratch_floats = align64f(plan_scratch_floats(pv, flags, chunk_max));
-  auto block_taps = [&](const cistgcn_block_taps& src, const int32_t* bd, long long s) {
-    cistgcn_block_taps bt = {nullptr, nullptr, nullptr, nullptr};
-    const size_t tv = (size_t)bd[CB_T] * bd[CB_V];
-    bt.adj_s = src.adj_s ? src.adj_s + (size_t)s * tv * bd[CB_T] : nullptr;
-    bt.adj_t = src.adj_t ? src.adj_t + (size_t)s * tv * bd[CB_V] : nullptr;
-    bt.w1 = src.w1 ? src.w1 + (size_t)s * bd[CB_CO] : nullptr;
-    bt.w2 = src.w2 ? src.w2 + (size_t)s * bd[CB_CO] : nullptr;
-    return bt;
-  };
+  const ChunkWorkspace w = chunk_workspace(pv, plan, chunk_max, workspace);
   for (long long s = 0; s < batch; s += chunk_max) {
     const long long n = (batch - s) < chunk_max ? (batch - s) : chunk_max;
-    const float* xs = x + (size_t)s * T * V * 3;
-    const float* cur = xs;
-    float* bufs[2] = {act0, act1};
-    int flip = 0;
-    for (int i = 0; i < pv.n_in; ++i) {
-      const int32_t* bd = pv.in_blocks + i * CB_COUNT;
-      cistgcn_block_taps bt = {nullptr, nullptr, nullptr, nullptr};
-      if (taps) bt = block_taps(taps->in_blocks[i], bd, s);
-      float* dst = bufs[flip];
-      // bf16 forward: every inter-block activation of the input stack (and the FPN's input) is stored as bf16
-      if (int rc = launch_dstd(bd, weights, cur, dst, n, taps ? &bt : nullptr, scratch, scratch_floats, flags, stream,
-                               act_bf16 && i > 0, act_bf16))
-        return rc;
-      cur = dst;
-      flip ^= 1;
-    }
-    if (int rc = launch_fpn(pv.fpn, pv.n_fpn, pv.tail, weights, cur, x7, n, flags, stream, act_bf16)) return rc;
-    cur = x7;
-    for (int i = 0; i < pv.n_out; ++i) {
-      const int32_t* bd = pv.out_blocks + i * CB_COUNT;
-      cistgcn_block_taps bt = {nullptr, nullptr, nullptr, nullptr};
-      if (taps) bt = block_taps(taps->out_blocks[i], bd, s);
-      float* dst = (i == pv.n_out - 1) ? x8 : bufs[flip];
-      if (int rc = launch_dstd(bd, weights, cur, dst, n, taps ? &bt : nullptr, scratch, scratch_floats, flags, stream)) return rc;
-      cur = dst;
-      flip ^= 1;
-    }
-    if (int rc = launch_tail(pv.tail, weights, xs, x7, x8, pred + (size_t)s * To * V * 3,
-                             target ? target + (size_t)s * To * V * 3 : nullptr, frame_sums, n, taps, s, stream))
+    if (int rc = forward_chunk(pv, weights, x + (size_t)s * T * V * 3, pred + (size_t)s * To * V * 3,
+                               target ? target + (size_t)s * To * V * 3 : nullptr, frame_sums, n, taps, s, w, flags,
+                               stream, act_bf16))
       return rc;
   }
   return 0;
@@ -605,6 +631,68 @@ int cistgcn_forward_bf16(const int32_t* plan, int32_t plan_len, const float* wei
                          const float* target, double* frame_sums, void* workspace, size_t workspace_bytes,
                          int64_t batch, const cistgcn_taps* taps, void* stream) {
   return forward_impl(plan, plan_len, weights, x, pred, target, frame_sums, workspace, workspace_bytes, batch, taps, stream, true);
+}
+
+// rollout workspace per chunk: the forward's, then [window (Tin frames)][step prediction (Tout frames)], 256-byte aligned
+size_t cistgcn_rollout_workspace_bytes(const int32_t* plan, int64_t batch) {
+  const size_t fwd = cistgcn_workspace_bytes(plan, batch);
+  if (!fwd) return 0;
+  const long long chunk = batch < CISTGCN_MAX_CHUNK ? (batch > 0 ? batch : 1) : CISTGCN_MAX_CHUNK;
+  const size_t pose = (size_t)chunk * plan[CP_V] * 3;
+  return fwd + (align64f(pose * plan[CP_TIN]) + align64f(pose * plan[CP_TOUT])) * sizeof(float);
+}
+
+// K = ceil(horizon / Tout) forwards per chunk, back to back on the caller's stream; step k reads the window written by
+// step k - 1 (the chunk's x for k = 0) and rollout_step_kernel scatters its prediction
+static int rollout_impl(const int32_t* plan, int32_t plan_len, const float* weights, const float* x, int32_t horizon,
+                        float* out, const float* target, double* frame_sums, void* workspace, size_t workspace_bytes,
+                        int64_t batch, void* stream, bool act_bf16) {
+  PlanView pv;
+  if (int rc = parse_plan(plan, plan_len, pv)) return rc;
+  if (batch < 0) return fail(-1, "negative batch");
+  if (horizon < 1) return fail(-1, "rollout: horizon = %d, must be >= 1", horizon);
+  if (batch == 0) return 0;
+  if (!weights || !x || !out || !workspace) return fail(-1, "NULL buffer");
+  if ((target == nullptr) != (frame_sums == nullptr)) return fail(-1, "target and frame_sums must be given together");
+  const size_t need = cistgcn_rollout_workspace_bytes(plan, batch);
+  if (workspace_bytes < need) return fail(-1, "rollout: workspace too small (%zu bytes given, %zu needed)", workspace_bytes, need);
+  const uint32_t flags = (uint32_t)plan[CP_FLAGS];
+  const int T = plan[CP_TIN], To = plan[CP_TOUT], V = plan[CP_V];
+  const long long chunk_max = batch < CISTGCN_MAX_CHUNK ? batch : CISTGCN_MAX_CHUNK;
+  const ChunkWorkspace w = chunk_workspace(pv, plan, chunk_max, workspace);
+  float* window = w.end;
+  float* step = window + align64f((size_t)chunk_max * T * V * 3);
+  const int K = (horizon + To - 1) / To;
+  for (long long s = 0; s < batch; s += chunk_max) {
+    const long long n = (batch - s) < chunk_max ? (batch - s) : chunk_max;
+    const float* in = x + (size_t)s * T * V * 3;
+    for (int k = 0; k < K; ++k) {
+      if (int rc = forward_chunk(pv, weights, in, step, nullptr, nullptr, n, nullptr, 0, w, flags, stream, act_bf16)) return rc;
+      const int t0 = k * To, nf = horizon - t0 < To ? horizon - t0 : To;
+      int e;
+      { ProfScope prof(KIND_OTHER, stream);
+        e = cg::launch_rollout_step(step, out + (size_t)s * horizon * V * 3, k + 1 < K ? window : nullptr,
+                                    target ? target + (size_t)s * horizon * V * 3 : nullptr, frame_sums, n, t0, nf,
+                                    horizon, T, To, V, stream); }
+      if (e) return check_launch(e, "rollout_step_kernel");
+      in = window;
+    }
+  }
+  return 0;
+}
+
+int cistgcn_rollout_f32(const int32_t* plan, int32_t plan_len, const float* weights, const float* x, int32_t horizon,
+                        float* out, const float* target, double* frame_sums, void* workspace, size_t workspace_bytes,
+                        int64_t batch, void* stream) {
+  return rollout_impl(plan, plan_len, weights, x, horizon, out, target, frame_sums, workspace, workspace_bytes, batch,
+                      stream, false);
+}
+
+int cistgcn_rollout_bf16(const int32_t* plan, int32_t plan_len, const float* weights, const float* x, int32_t horizon,
+                         float* out, const float* target, double* frame_sums, void* workspace, size_t workspace_bytes,
+                         int64_t batch, void* stream) {
+  return rollout_impl(plan, plan_len, weights, x, horizon, out, target, frame_sums, workspace, workspace_bytes, batch,
+                      stream, true);
 }
 
 size_t cistgcn_dstd_block_workspace_bytes(const int32_t* block_desc, int64_t batch) {

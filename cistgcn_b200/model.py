@@ -15,6 +15,7 @@ from __future__ import annotations
 
 import copy
 import ctypes
+import operator
 import time
 import warnings
 from typing import Dict, List, Optional, Tuple
@@ -397,6 +398,59 @@ class CISTGCN(nn.Module):
                 or target.device != x.device:
             raise ValueError("cistgcn_b200: target must be (B, output_n, joints, 3) float32 on x's device")
         return self._run(x, target.contiguous())
+
+    def rollout(self, x, horizon) -> torch.Tensor:
+        """Autoregressive forecast past output_n, eval mode only: ceil(horizon / output_n) forwards, each fed the last
+        input_n frames of the previous prediction (the first one x).  Returns (B, horizon, joints, 3) = the concatenated
+        predictions cut to `horizon`, bit-identical to that loop over ``model(...)`` at the same batch size."""
+        return self._rollout(x, horizon, None)[0]
+
+    def rollout_mpjpe(self, x, target):
+        """``rollout(x, target.shape[1])`` + fused MPJPE partial sums: returns (pred, frame_sums), frame_sums a float64
+        (horizon,) tensor with the meaning of ``forward_mpjpe``'s, so it plugs into ``dist.sharded_eval_mpjpe``."""
+        if not isinstance(target, torch.Tensor) or target.dim() != 4:
+            raise ValueError("cistgcn_b200: target must be a (B, horizon, joints, 3) tensor")
+        return self._rollout(x, target.shape[1], target)
+
+    def _rollout(self, x, horizon, target):
+        if self.training:
+            raise ValueError("cistgcn_b200: rollout runs in eval mode only (call model.eval())")
+        if torch.is_grad_enabled() and getattr(x, "requires_grad", False):
+            raise ValueError("cistgcn_b200: rollout is not differentiable; loop forward() for input gradients")
+        if isinstance(horizon, bool):
+            horizon = None
+        try:
+            horizon = operator.index(horizon)
+        except TypeError:
+            horizon = None
+        if horizon is None or not 1 <= horizon < 2**31:
+            raise ValueError("cistgcn_b200: horizon must be an integer >= 1")
+        if target is not None:
+            B = x.shape[0] if isinstance(x, torch.Tensor) else None
+            if target.shape != (B, horizon, self.n_joints, 3) or target.dtype != torch.float32 \
+                    or target.device != getattr(x, "device", None):
+                raise ValueError("cistgcn_b200: target must be (B, horizon, joints, 3) float32 on x's device")
+            target = target.contiguous()
+        self._check_input(x)
+        lib = _cabi.lib()
+        x = x.contiguous()
+        B = x.shape[0]
+        packed = self.pack(x.device)
+        packed.plan_c[F["CP_FLAGS"]] = int(self.kernel_flags)
+        out = torch.empty(B, horizon, self.n_joints, 3, device=x.device, dtype=torch.float32)
+        sums = torch.zeros(horizon, device=x.device, dtype=torch.float64) if target is not None else None
+        if B == 0:
+            return out, sums
+        workspace = torch.empty(lib.cistgcn_rollout_workspace_bytes(packed.plan_c, B), device=x.device, dtype=torch.uint8)
+        stream = torch.cuda.current_stream(x.device).cuda_stream
+        name = "cistgcn_rollout_bf16" if self.act_dtype == torch.bfloat16 else "cistgcn_rollout_f32"
+        with torch.cuda.device(x.device):
+            rc = getattr(lib, name)(packed.plan_c, len(packed.plan), packed.blob.data_ptr(), x.data_ptr(), horizon,
+                                    out.data_ptr(), target.data_ptr() if target is not None else None,
+                                    sums.data_ptr() if sums is not None else None,
+                                    workspace.data_ptr(), workspace.numel(), B, stream)
+        _cabi.check(rc, name)
+        return out, sums
 
     def _run(self, x, target):
         self._check_input(x)

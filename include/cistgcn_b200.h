@@ -17,6 +17,8 @@
  *   cistgcn_forward_bf16
  *                            environment/train.py:59 and environment/test.py:101,103
  *                            (+ losses/losses.py:50-61 mpjpe when `target` is given)
+ *   cistgcn_rollout_f32 /    no counterpart: the autoregressive loop a caller writes around CISTGCN.forward to reach
+ *   cistgcn_rollout_bf16     horizons past output_n (+ losses.mpjpe over the whole horizon when `target` is given)
  *   cistgcn_dstd_block_f32   models/CISTGCN/CISTGCN.py:373-390  DSTD_GC.forward (one block)
  *   cistgcn_fpn_chain_f32    models/CISTGCN/CISTGCN.py:582-589  FPN stack + dim_conversor + cumsum
  *   cistgcn_tail_f32         models/CISTGCN/CISTGCN.py:591-597  ContextLayer + output assembly
@@ -221,6 +223,23 @@ int cistgcn_forward_bf16(const int32_t* plan, int32_t plan_len, const float* wei
                          const float* x, float* pred, const float* target, double* frame_sums,
                          void* workspace, size_t workspace_bytes, int64_t batch,
                          const cistgcn_taps* taps, void* stream);
+
+/* Autoregressive rollout to `horizon` >= 1 frames: K = ceil(horizon / Tout) forwards per chunk of CISTGCN_MAX_CHUNK
+ * samples, back to back on `stream` (no host synchronisation).  Step 0 reads x (B, Tin, V, 3); step k + 1 reads the last
+ * Tin frames of step k's prediction p_k (Tin <= Tout, so exactly p_k[:, Tout - Tin:]).  out (B, horizon, V, 3):
+ * p_0, ..., p_{K-1} concatenated along the frames and cut to `horizon`, bit-identical to the same loop over
+ * cistgcn_forward_f32 (_bf16) at the same batch size.  target (optional, same shape as out) + frame_sums (optional, double[horizon], ACCUMULATED into):
+ * per-frame sums of ||out - target||_2 as in cistgcn_forward_f32.  No taps.  Unsupported shapes fail as in the
+ * forward, before anything is written.  The workspace is the forward's plus one window and one step prediction per
+ * chunk: cistgcn_rollout_workspace_bytes(plan, batch) bytes. */
+size_t cistgcn_rollout_workspace_bytes(const int32_t* plan, int64_t batch);
+int cistgcn_rollout_f32(const int32_t* plan, int32_t plan_len, const float* weights, const float* x,
+                        int32_t horizon, float* out, const float* target, double* frame_sums,
+                        void* workspace, size_t workspace_bytes, int64_t batch, void* stream);
+/* Same with the bf16 activation storage of cistgcn_forward_bf16. */
+int cistgcn_rollout_bf16(const int32_t* plan, int32_t plan_len, const float* weights, const float* x,
+                         int32_t horizon, float* out, const float* target, double* frame_sums,
+                         void* workspace, size_t workspace_bytes, int64_t batch, void* stream);
 
 /* One DSTD-GC block on `batch` samples with the strides in the descriptor.  The three-stage path needs
  * cistgcn_dstd_block_workspace_bytes(desc, batch) bytes of scratch (stage records + gates + adjacencies). */
