@@ -87,6 +87,12 @@ def bind(path: str) -> ctypes.CDLL:
     L.cistgcn_eval_metrics_f32.restype = ctypes.c_int
     L.cistgcn_eval_metrics_f32.argtypes = [_p, _p, _p, _p, ctypes.c_int32, _p, _p, _p, _p, ctypes.c_int64, ctypes.c_int32,
                                            ctypes.c_int32, ctypes.c_int32, _p]
+    L.cistgcn_mpjpe_grouped_f32.restype = ctypes.c_int
+    L.cistgcn_mpjpe_grouped_f32.argtypes = [_p, _p, _p, ctypes.c_int32, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, _p, _p,
+                                            _p]
+    L.cistgcn_eval_metrics_grouped_f32.restype = ctypes.c_int
+    L.cistgcn_eval_metrics_grouped_f32.argtypes = [_p, _p, _p, ctypes.c_int32, _p, _p, ctypes.c_int32, _p, _p, _p, _p, _p,
+                                                   ctypes.c_int64, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _p]
     L.cistgcn_augment_windows_f32.restype = ctypes.c_int
     L.cistgcn_augment_windows_f32.argtypes = [_p, _p, _p, _p, _p, _p, _p, _p, _p, ctypes.c_int64, ctypes.c_int32, ctypes.c_int32,
                                               ctypes.c_int32, _p]

@@ -25,6 +25,9 @@ namespace cg {
 // csrc/rollout.cu: moves one rollout step's prediction into the output and the next input window; 0 or a CUDA error
 int launch_rollout_step(const float* pred, float* out, float* window, const float* target, double* frame_sums,
                         long long n, int t0, int nf, int H, int Tin, int To, int V, void* stream);
+// csrc/eval_grouped.cu: per-group per-frame MPJPE sums and sample counts; 0 or a CUDA error
+int launch_mpjpe_grouped(const float* pred, const float* target, const int* groups, int G, long long batch, int T, int V,
+                         double* sums, long long* counts, void* stream);
 }  // namespace cg
 
 namespace {
@@ -37,7 +40,7 @@ constexpr int kMaxSmemBytes = 227 * 1024;
 
 namespace cgt {
 // Records the message for cistgcn_last_error() and returns code: the error sink of every entry point, also those of
-// train_ops.cu, augment.cu and eval_metrics.cu
+// train_ops.cu, augment.cu, eval_metrics.cu and eval_grouped.cu
 int fail_train(int code, const char* fmt, ...) {
   char buf[512];
   va_list ap;
@@ -745,6 +748,17 @@ int cistgcn_mpjpe_f32(const float* pred, const float* target, int64_t batch, int
   ProfScope prof(KIND_MPJPE, stream);
   CG_LAUNCH(kfn, (int)(blocks < cap ? blocks : cap), 256, 0, stream, a);
   return check_launch(cg::last_launch_error(), "mpjpe_kernel");
+}
+
+int cistgcn_mpjpe_grouped_f32(const float* pred, const float* target, const int32_t* groups, int32_t n_groups, int64_t batch,
+                              int32_t T, int32_t V, double* sums, int64_t* counts, void* stream) {
+  if (!pred || !target || !sums || !counts) return fail(-1, "mpjpe_grouped: NULL buffer");
+  if (n_groups < 1 || T < 1 || V < 1 || (long long)n_groups * T > 0x7fffffffLL)
+    return fail(-1, "mpjpe_grouped: n_groups = %d, T = %d, V = %d must be positive (n_groups * T < 2^31)", n_groups, T, V);
+  if (batch <= 0) return batch == 0 ? 0 : fail(-1, "negative batch");
+  ProfScope prof(KIND_MPJPE, stream);
+  return check_launch(cg::launch_mpjpe_grouped(pred, target, groups, n_groups, batch, T, V, sums,
+                                               reinterpret_cast<long long*>(counts), stream), "grouped_mpjpe_kernel");
 }
 
 }  // extern "C"

@@ -4,7 +4,8 @@ Samples are independent in eval mode, so inference shards the batch by rank with
 collective: every rank (one process per GPU, launched by torchrun) runs the fused forward on its own
 contiguous chunk.  The only exchange is the MPJPE bookkeeping: per-frame error sums (output_n doubles
 = 200 bytes) are summed over ranks once per evaluation -- `torch.distributed.all_reduce`, which is NCCL
-over NVLink on the GPU box and gloo in the CPU tests.
+over NVLink on the GPU box and gloo in the CPU tests.  Grouped evaluation (one row per action or
+sub-dataset, `sharded_eval_grouped`) exchanges G*T frame sums and G sample counts in one all-reduce.
 """
 from __future__ import annotations
 
@@ -52,3 +53,41 @@ def sharded_eval_mpjpe(forward_mpjpe: Callable, x: torch.Tensor, target: torch.T
     tot, cnt = combine_frame_sums(sums, (hi - lo) * V, group)
     per_frame = tot / max(cnt, 1)
     return pred, (lo, hi), per_frame.mean(), per_frame
+
+
+def sharded_eval_grouped(fn: Callable, x: torch.Tensor, target: torch.Tensor, groups: torch.Tensor, n_groups: int,
+                         rank: Optional[int] = None, world: Optional[int] = None, group=None):
+    """Per-group per-frame MPJPE of a global batch held by every rank (e.g. one row per H3.6M action): each rank
+    processes only its contiguous shard with the matching slice of `groups`.
+
+    fn(x_shard, target_shard, groups_shard, n_groups) -> (pred_shard, sums (G, T), counts (G,)) -- normally
+    CISTGCN.forward_mpjpe or CISTGCN.rollout_mpjpe.  The sums and counts of all ranks are combined in ONE all-reduce of
+    G*T + G doubles.  Returns (pred_shard, (lo, hi), per_group_per_frame (G, T) float64, counts (G,) int64), where row g
+    is losses.mpjpe(..., reduce_axis=(0, 2)) over group g's samples (NaN for a group without samples).  Raises
+    ValueError when the global counts do not add up to the global batch (ids outside [0, n_groups))."""
+    if rank is None:
+        rank = dist.get_rank(group) if dist.is_initialized() else 0
+    if world is None:
+        world = dist.get_world_size(group) if dist.is_initialized() else 1
+    B = x.shape[0]
+    if not isinstance(groups, torch.Tensor) or groups.shape != (B,):
+        raise ValueError("sharded_eval_grouped: groups must be a (B,) tensor of group ids")
+    lo, hi = shard_bounds(B, rank, world)
+    V, T = target.shape[2], target.shape[1]
+    if hi > lo:
+        pred, sums, counts = fn(x[lo:hi].contiguous(), target[lo:hi].contiguous(), groups[lo:hi], n_groups)
+    else:
+        pred = target[lo:hi]
+        sums = torch.zeros(n_groups, T, dtype=torch.float64, device=x.device)
+        counts = torch.zeros(n_groups, dtype=torch.int64, device=x.device)
+    buf = torch.cat([sums.to(torch.float64).reshape(-1), counts.to(sums.device, torch.float64)])
+    if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+    tot = buf[:-n_groups].view(n_groups, T)
+    cnt = buf[-n_groups:].round().to(torch.int64)
+    n = int(cnt.sum())
+    if n != B:
+        raise ValueError(f"sharded_eval_grouped: the groups count {n} samples, the batch has {B} "
+                         f"(group ids outside [0, {n_groups})?)")
+    per = torch.where(cnt[:, None] > 0, tot / (cnt[:, None].to(torch.float64) * V).clamp(min=1), float("nan"))
+    return pred, (lo, hi), per, cnt

@@ -390,14 +390,25 @@ class CISTGCN(nn.Module):
         pred, _ = self._run(x, None)
         return pred,                                         # 1-tuple, like CISTGCN.py:597
 
-    def forward_mpjpe(self, x, target):
+    def forward_mpjpe(self, x, target, groups=None, n_groups=None):
         """Forward + fused MPJPE partial sums.  Returns (pred, frame_sums) where frame_sums is a
         float64 (output_n,) tensor: sum over samples and joints of ||pred - target||_2 per frame.
-        mpjpe(reduce_axis=[]) = frame_sums.sum() / (B*T*V); (0,2) = frame_sums / (B*V)."""
+        mpjpe(reduce_axis=[]) = frame_sums.sum() / (B*T*V); (0,2) = frame_sums / (B*V).
+
+        With ``groups`` (a (B,) integer tensor of per-sample group ids, e.g. the action of every window) and
+        ``n_groups``: returns (pred, sums, counts) instead, sums a float64 (n_groups, output_n) tensor of the same frame
+        sums per group and counts an int64 (n_groups,) tensor of samples per group, so group g's per-frame MPJPE is
+        sums[g] / (counts[g] * joints).  ``pred`` is ``forward(x)[0]``; the sums come from one extra pass over pred and
+        target.  A CPU ``groups`` tensor is range-checked here (ValueError); ids of a CUDA ``groups`` tensor are not
+        (that would synchronise): samples whose id is outside [0, n_groups) are left out of sums and counts."""
         if target.shape != (x.shape[0], self.n_output, self.n_joints, 3) or target.dtype != torch.float32 \
                 or target.device != x.device:
             raise ValueError("cistgcn_b200: target must be (B, output_n, joints, 3) float32 on x's device")
-        return self._run(x, target.contiguous())
+        if groups is None and n_groups is None:
+            return self._run(x, target.contiguous())
+        groups = self._check_groups(groups, n_groups, x)
+        pred = self._run(x, None)[0]
+        return (pred,) + self._grouped_mpjpe(pred, target, groups, n_groups)
 
     def rollout(self, x, horizon) -> torch.Tensor:
         """Autoregressive forecast past output_n, eval mode only: ceil(horizon / output_n) forwards, each fed the last
@@ -405,12 +416,59 @@ class CISTGCN(nn.Module):
         predictions cut to `horizon`, bit-identical to that loop over ``model(...)`` at the same batch size."""
         return self._rollout(x, horizon, None)[0]
 
-    def rollout_mpjpe(self, x, target):
+    def rollout_mpjpe(self, x, target, groups=None, n_groups=None):
         """``rollout(x, target.shape[1])`` + fused MPJPE partial sums: returns (pred, frame_sums), frame_sums a float64
-        (horizon,) tensor with the meaning of ``forward_mpjpe``'s, so it plugs into ``dist.sharded_eval_mpjpe``."""
+        (horizon,) tensor with the meaning of ``forward_mpjpe``'s, so it plugs into ``dist.sharded_eval_mpjpe``.
+        With ``groups`` / ``n_groups``: returns (pred, sums (n_groups, horizon), counts (n_groups,)) as ``forward_mpjpe``
+        does, so it plugs into ``dist.sharded_eval_grouped``."""
         if not isinstance(target, torch.Tensor) or target.dim() != 4:
             raise ValueError("cistgcn_b200: target must be a (B, horizon, joints, 3) tensor")
-        return self._rollout(x, target.shape[1], target)
+        if groups is None and n_groups is None:
+            return self._rollout(x, target.shape[1], target)
+        B = x.shape[0] if isinstance(x, torch.Tensor) else None
+        if target.shape != (B, target.shape[1], self.n_joints, 3) or target.dtype != torch.float32 \
+                or target.device != getattr(x, "device", None):
+            raise ValueError("cistgcn_b200: target must be (B, horizon, joints, 3) float32 on x's device")
+        groups = self._check_groups(groups, n_groups, x)
+        pred = self._rollout(x, target.shape[1], None)[0]
+        return (pred,) + self._grouped_mpjpe(pred, target, groups, n_groups)
+
+    def _check_groups(self, groups, n_groups, x):
+        """Validates per-sample group ids before the library is reached; returns them as int32 on x's device."""
+        if isinstance(n_groups, bool):
+            n_groups = None
+        try:
+            n_groups = operator.index(n_groups)
+        except TypeError:
+            n_groups = None
+        if n_groups is None or not 1 <= n_groups < 2**31:
+            raise ValueError("cistgcn_b200: n_groups must be an integer >= 1 when groups are given")
+        B = x.shape[0] if isinstance(x, torch.Tensor) else None
+        if not isinstance(groups, torch.Tensor) or groups.shape != (B,) or groups.is_floating_point() \
+                or groups.is_complex() or groups.dtype == torch.bool:
+            raise ValueError("cistgcn_b200: groups must be a (B,) integer tensor of group ids")
+        if groups.is_cuda:
+            if groups.device != x.device:
+                raise ValueError("cistgcn_b200: groups must live on the CPU or on x's device")
+        elif groups.numel() and (int(groups.min()) < 0 or int(groups.max()) >= n_groups):
+            raise ValueError(f"cistgcn_b200: group ids must lie in [0, {n_groups})")
+        return groups.to(x.device, torch.int32).contiguous()
+
+    def _grouped_mpjpe(self, pred, target, groups, n_groups):
+        """(sums (G, T) float64, counts (G,) int64) of cistgcn_mpjpe_grouped_f32 over pred / target."""
+        B, T, V, _ = pred.shape
+        sums = torch.zeros(n_groups, T, device=pred.device, dtype=torch.float64)
+        counts = torch.zeros(n_groups, device=pred.device, dtype=torch.int64)
+        if B == 0:
+            return sums, counts
+        lib = _cabi.lib()
+        pred_c, target = pred.detach().contiguous(), target.contiguous()
+        stream = torch.cuda.current_stream(pred.device).cuda_stream
+        with torch.cuda.device(pred.device):
+            rc = lib.cistgcn_mpjpe_grouped_f32(pred_c.data_ptr(), target.data_ptr(), groups.data_ptr(), n_groups, B, T, V,
+                                               sums.data_ptr(), counts.data_ptr(), stream)
+        _cabi.check(rc, "cistgcn_mpjpe_grouped_f32")
+        return sums, counts
 
     def _rollout(self, x, horizon, target):
         if self.training:

@@ -23,6 +23,7 @@
  *   cistgcn_fpn_chain_f32    models/CISTGCN/CISTGCN.py:582-589  FPN stack + dim_conversor + cumsum
  *   cistgcn_tail_f32         models/CISTGCN/CISTGCN.py:591-597  ContextLayer + output assembly
  *   cistgcn_mpjpe_f32        losses/losses.py:50-61             mpjpe (all three reduce_axis modes)
+ *   cistgcn_mpjpe_grouped_f32  the same per-frame sums split by a per-sample group id (one row per action / sub-dataset)
  *
  * Descriptors are flat int32 arrays indexed by the enums below.  Weight fields are offsets (in
  * floats) into the packed weight blob produced by cistgcn_b200/pack.py (BatchNorm folded,
@@ -262,6 +263,15 @@ int cistgcn_tail_f32(const int32_t* tail_desc, const float* weights, const float
 int cistgcn_mpjpe_f32(const float* pred, const float* target, int64_t batch, int32_t T, int32_t V,
                       float* err, double* frame_sums, void* stream);
 
+/* Grouped mpjpe for per-group (per action, per sub-dataset) tables in one pass.  pred, target (B, T, V, 3); groups[B]
+ * int32 group id of every sample, or NULL = every sample in group 0.  ACCUMULATES into sums[n_groups][T] (double: sum over
+ * the group's samples and the joints of ||pred - target||_2 per frame, the scheme of cistgcn_mpjpe_f32) and counts[n_groups]
+ * (int64: samples).  Group g's per-frame MPJPE is sums[g] / (counts[g] * V).  A sample whose id is outside [0, n_groups)
+ * is skipped and not counted; nothing outside sums / counts is written.  -1: NULL pred / target / sums / counts,
+ * n_groups < 1, T < 1, V < 1, negative batch; batch 0 is a no-op.  Timed under the profile kind "mpjpe_kernel". */
+int cistgcn_mpjpe_grouped_f32(const float* pred, const float* target, const int32_t* groups, int32_t n_groups,
+                              int64_t batch, int32_t T, int32_t V, double* sums, int64_t* counts, void* stream);
+
 /* Fused evaluation metrics (environment/test.py:65-94 Metrics.compute, :125-129 the scatter of the model's joints into the
  * full skeleton).  pred (B, To, Vu, 3) = model output on the used joints; target (B, To, Vf, 3) = full skeleton;
  * src_map[Vf]: index into pred's joints or -1 (keep the target's joint: dim_used / dim_repeat_32 <- dim_repeat_22 of
@@ -281,6 +291,17 @@ enum cistgcn_metric {
 int cistgcn_eval_metrics_f32(const float* pred, const float* target, const int32_t* src_map, const int32_t* bones,
                              int32_t n_bones, const float* weights0, const float* weights1, float* assembled,
                              double* sums, int64_t batch, int32_t To, int32_t Vu, int32_t Vf, void* stream);
+/* Grouped form of cistgcn_eval_metrics_f32, with no limit on To (cistgcn_eval_metrics_f32 takes To <= 32).  groups[B]
+ * int32 group id of every sample, or NULL = every sample in group 0.  ACCUMULATES into sums[n_groups][CISTGCN_METRIC_COUNT][To]
+ * (each group's block means what cistgcn_eval_metrics_f32's sums mean for that group's samples) and counts[n_groups]
+ * (int64: samples).  A sample whose id is outside [0, n_groups) is skipped and not counted (its `assembled` rows are still
+ * written); nothing outside sums / counts / assembled is written.  -1: NULL pred / target / src_map / sums / counts,
+ * n_groups < 1, To < 1, joints out of range, negative batch; batch 0 is a no-op.  Not timed by cistgcn_profile_*, like
+ * cistgcn_eval_metrics_f32. */
+int cistgcn_eval_metrics_grouped_f32(const float* pred, const float* target, const int32_t* groups, int32_t n_groups,
+                                     const int32_t* src_map, const int32_t* bones, int32_t n_bones, const float* weights0,
+                                     const float* weights1, float* assembled, double* sums, int64_t* counts,
+                                     int64_t batch, int32_t To, int32_t Vu, int32_t Vf, void* stream);
 
 /* GPU-side training-batch pipeline (loaders/h36m_motion_3d.py:94-108 window split + velocity / speed targets;
  * environment/custom_transforms.py:10-419 RandomFlip, RandomRotation, RandomScale, RandomNoise, RandomTranslation in the
